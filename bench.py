@@ -236,6 +236,18 @@ def reference_gpu(w, iters, solver):
             "what": "unmodified aCG GPU solver (cuSPARSE SpMV, cuBLAS dot), 'total solver time' of its own report"}
 
 
+DUMP_ROWS = 1 << 21       # 2 x 16 MB of float64 at most, whatever the workload
+
+
+def dump_sample(x, rnrm2, r0nrm2):
+    """What a caller of the timed solve receives, as float64 arrays: x at a fixed, seeded sample of
+    DUMP_ROWS rows (every row of a smaller problem) with those row numbers, and ||r||, ||r0||."""
+    n = len(x)
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    return {"x": x[rows].astype(np.float64), "x_rows": rows.astype(np.float64),
+            "residual_norms": np.array([rnrm2, r0nrm2], dtype=np.float64)}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -253,7 +265,12 @@ def main():
                     help="also run the stock reference GPU solver (cuSPARSE/cuBLAS) on the same matrix (1 GPU, adds minutes)")
     ap.add_argument("--partition", default="block", choices=["block", "metis"],
                     help="row partition for N>1: geometric blocks or METIS (acgsymcsrmatrix_partition_rows)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (x at a fixed sample of rows, the solver's residual "
+                         "norms) as DIR/*.npy, to compare two builds output for output (1 GPU)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.gpus != 1 or args.impl != "acgb200" or args.steps < 1):
+        ap.error("--dump-outputs needs --gpus 1, --impl acgb200 and at least one step")
     # torchrun exports OMP_NUM_THREADS=1 to every rank unless the caller set it.  The host-side set-up
     # (matrix generator, full-storage expansion) is OpenMP code: give a rank of the GPU arm its share of
     # the host cores.  (The CPU arm sets its own OpenMP environment in its own process, oracle/cpu_arm.py.)
@@ -354,6 +371,8 @@ def main():
         inf = cg.info()
         dev_ms += inf["last_solve_ms"]
         launches += inf["last_launches"]
+    if args.dump_outputs:
+        dumped = dump_sample(x.x[:nown], cg.c.rnrm2, cg.c.r0nrm2)
     # ---- same steps again with a CUDA-event pair around every SpMV on its launching
     # stream (the library's profile mode; it issues the same kernels un-graphed)
     ab.set_option("profile", 1)
@@ -474,6 +493,10 @@ def main():
             cg.free(); b.free(); x.free(); A.free()          # give the memory back first
             line["reference_gpu"] = reference_gpu(w, args.iters, solver)
         print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     cg.free(); b.free(); x.free()
     comm.destroy()
     if world > 1:

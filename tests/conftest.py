@@ -1,4 +1,6 @@
 import glob
+import hashlib
+import json
 import os
 import sys
 
@@ -85,3 +87,17 @@ def ab():
 def load_golden(path):
     z = np.load(path)
     return {k: z[k] for k in z.files}
+
+
+def load_golden_json(name):
+    with open(os.path.join(ROOT, "tests", "golden", "reference", name + ".json")) as f:
+        return json.load(f)
+
+
+def digest(a):
+    """SHA-256 of an array's dtype, shape and bytes: what tests/golden/reference/*.json store in place
+    of arrays that are compared bit for bit, to keep the fixtures small."""
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(f"{a.dtype.str}{a.shape}".encode())
+    h.update(a.tobytes())
+    return h.hexdigest()

@@ -1,6 +1,7 @@
 """The C-ABI boundary: library loads, exports what include/ declares, and its
-struct layouts are the reference's (checked by compiling the same probe against
-/root/reference's headers and against include/acgb200/)."""
+struct layouts are the reference's (the same probe compiled against
+include/acgb200/ prints what it printed compiled against the reference's
+headers, tests/golden/reference/struct_layouts.txt)."""
 import ctypes
 import glob
 import os
@@ -8,10 +9,7 @@ import re
 import subprocess
 import tempfile
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 PROBE = r"""
 #include <stddef.h>
@@ -71,13 +69,12 @@ def test_error_strings(ab):
     assert b"NVSHMEM" in L.acgerrcodestr(16, 0)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF + "/acg"), reason="reference tree not present (GPU box)")
 def test_struct_layouts_match_reference_headers():
     cuda_inc = "/usr/local/cuda/include"
     mine = _run_probe('#include "acgb200/cgcuda.h"\n#include "acgb200/error.h"',
                       ["-I" + os.path.join(ROOT, "include"), "-I" + cuda_inc])
-    theirs = _run_probe('#include "acg/vector.h"\n#include "acg/graph.h"\n#include "acg/symcsrmatrix.h"\n'
-                        '#include "acg/cgcuda.h"\n#include "acg/error.h"', ["-I" + REF])
+    with open(os.path.join(ROOT, "tests", "golden", "reference", "struct_layouts.txt")) as f:
+        theirs = f.read()
     assert mine == theirs
 
 

@@ -188,15 +188,17 @@ CONTRACT_KEYS = ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per
 
 
 @pytest.mark.parametrize("nproc", [1, 2])
-def test_bench_main_runs_and_prints_the_contract_line(nproc, simlib):
+def test_bench_main_runs_and_prints_the_contract_line(nproc, simlib, tmp_path):
     """bench.py's main(), unchanged, on the stand-in (tests/hostsim/run_bench_sim.py patches
     torch.cuda availability and the nvidia-smi sampler around it): matrix set-up for one and
     several ranks, timed pass, profiled pass, one JSON line from rank 0 with every key of the
-    bench contract.  Shape only -- nothing it prints is a measurement."""
+    bench contract; on one rank, the outputs of the last timed step under --dump-outputs.
+    Shape only -- nothing it prints is a measurement."""
     script = os.path.join(SIM, "run_bench_sim.py")
     args = ["--gpus", str(nproc), "--workload", "27pt-64", "--steps", "2", "--warmup", "1", "--iters", "6", "--cpu-iters", "2"]
+    dump = str(tmp_path / "out")
     if nproc == 1:
-        cmd = [sys.executable, script] + args
+        cmd = [sys.executable, script] + args + ["--dump-outputs", dump]
     else:
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={nproc}",
                "--master-addr", "127.0.0.1", "--master-port", str(_free_port()), script] + args
@@ -219,6 +221,14 @@ def test_bench_main_runs_and_prints_the_contract_line(nproc, simlib):
     assert ("cpu_baseline" in d) == (nproc == 1)
     if nproc == 1:
         assert d["cpu_baseline"]["kind"] in ("reference", "port") and d["cpu_baseline"]["value"] > 0
+        import numpy as np
+        out = {k: np.load(os.path.join(dump, k + ".npy")) for k in ("x", "x_rows", "residual_norms")}
+        assert sorted(os.listdir(dump)) == ["residual_norms.npy", "x.npy", "x_rows.npy"]
+        assert all(a.dtype == np.float64 for a in out.values())
+        assert np.array_equal(out["x_rows"], np.arange(64 ** 3)) and out["x"].shape == (64 ** 3,)
+        assert np.isfinite(out["x"]).all() and np.abs(out["x"]).max() > 0
+        rn, r0 = out["residual_norms"]
+        assert rn / r0 == pytest.approx(d["residual_after_step"], rel=1e-12)
     else:
         assert d["config"]["partition"].startswith("2 parts")
 

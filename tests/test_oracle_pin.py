@@ -1,7 +1,9 @@
 """The oracle (oracle/cg_oracle.c) against the reference's own code and vectors.
 
-* bit-for-bit against oracle/_ref/libacgref.so (the unmodified reference
-  sources, compiled with -ffp-contract=off like the oracle) on seeded inputs;
+* bit-for-bit against what oracle/_ref/libacgref.so (the unmodified reference
+  sources, compiled with -ffp-contract=off like the oracle) computed on seeded
+  inputs, stored in tests/golden/reference/oracle_pin.json as scalars and
+  array digests (tools/make_reference_golden.py);
 * bit-for-bit against the committed fixtures tests/golden/*.npz, which were
   produced by that library alone (tools/make_golden.py);
 * the known-answer tests SURVEY.md §8(c) lists (KAT-1, KAT-2, KAT-3, KAT-6).
@@ -12,7 +14,7 @@ import numpy as np
 import pytest
 
 from acg_b200 import matgen as mg
-from conftest import GOLDEN, load_golden
+from conftest import GOLDEN, digest, load_golden, load_golden_json
 
 CASES = [
     ("27pt", lambda: mg.stencil3d_27pt(8)),
@@ -25,36 +27,39 @@ CASES = [
 ]
 
 
+@pytest.fixture(scope="module")
+def pin():
+    return load_golden_json("oracle_pin")
+
+
 @pytest.mark.parametrize("name,gen", CASES, ids=[c[0] for c in CASES])
-def test_oracle_equals_reference_bitwise(name, gen, oracle, ref):
+def test_oracle_equals_reference_bitwise(name, gen, oracle, pin):
     n, r, c, v = gen()
     csr_o = oracle.full_csr(n, r, c, v)
-    csr_r = ref.full_csr(n, r, c, v)
-    for a, b in zip(csr_o, csr_r):
-        assert np.array_equal(a, b)
+    for a, k in zip(csr_o, ("frowptr", "fcolidx", "fa")):
+        assert digest(a) == pin[f"{name}__{k}"], k
     rng = np.random.default_rng(1)
     x, y = rng.standard_normal(n), rng.standard_normal(n)
     # the two uses in acg/cg.c: r -= A x (alpha=-1,beta=1) and t = A p (alpha=1,beta=0)
-    for alpha, beta in ((-1.0, 1.0), (1.0, 0.0), (0.5, 2.0)):
-        assert np.array_equal(oracle.dsymv(csr_o, alpha, x, beta, y), ref.dsymv(n, r, c, v, alpha, x, beta, y))
-    assert oracle.ddot(x, y) == ref.ddot(x, y)
-    assert oracle.dnrm2sqr(x) == ref.dnrm2sqr(x)
+    for i, (alpha, beta) in enumerate(((-1.0, 1.0), (1.0, 0.0), (0.5, 2.0))):
+        assert digest(oracle.dsymv(csr_o, alpha, x, beta, y)) == pin[f"{name}__dsymv{i}"]
+    assert oracle.ddot(x, y) == pin[f"{name}__ddot"]
+    assert oracle.dnrm2sqr(x) == pin[f"{name}__dnrm2sqr"]
     b = rng.standard_normal(n)
-    for maxits, rtol in ((7, 0.0), (200, 1e-9)):
+    for i, (maxits, rtol) in enumerate(((7, 0.0), (200, 1e-9))):
         o = oracle.cg(csr_o, b, maxits=maxits, rtol=rtol)
-        f = ref.cg(n, r, c, v, b, maxits=maxits, rtol=rtol)
-        assert (o["status"], o["niterations"]) == (f["status"], f["niterations"])
-        assert np.array_equal(o["x"], f["x"])
-        assert (o["bnrm2"], o["r0nrm2"], o["rnrm2"]) == (f["bnrm2"], f["r0nrm2"], f["rnrm2"])
+        for k in ("status", "niterations", "bnrm2", "r0nrm2", "rnrm2"):
+            assert o[k] == pin[f"{name}__cg{i}__{k}"], k
+        assert digest(o["x"]) == pin[f"{name}__cg{i}__x"]
 
 
-def test_unsorted_coo_input(oracle, ref):
+def test_unsorted_coo_input(oracle, pin):
     """acg/symcsrmatrix.c:133-141: unsorted input takes the scatter branch."""
     n, r, c, v = mg.stencil3d_27pt(5)
     perm = np.random.default_rng(3).permutation(len(v))
     r2, c2, v2 = (np.ascontiguousarray(a[perm]) for a in (r, c, v))
-    for a, b in zip(oracle.full_csr(n, r2, c2, v2), ref.full_csr(n, r2, c2, v2)):
-        assert np.array_equal(a, b)
+    for a, k in zip(oracle.full_csr(n, r2, c2, v2), ("frowptr", "fcolidx", "fa")):
+        assert digest(a) == pin[f"unsorted__{k}"], k
 
 
 @pytest.mark.parametrize("path", GOLDEN, ids=[os.path.basename(p)[:-4] for p in GOLDEN])
@@ -112,19 +117,19 @@ def test_kat6_pipelined_tracks_classic(oracle):
     assert np.abs(a["x"] - p["x"]).max() <= 1e-9 * np.abs(a["x"]).max()
 
 
-def test_status_codes_and_edge_cases(oracle, ref):
+def test_status_codes_and_edge_cases(oracle, pin):
     n, r, c, v = mg.stencil3d_27pt(6)
     csr = oracle.full_csr(n, r, c, v)
     b = np.ones(n)
     # maxits only -> success; tolerance not met -> ACG_ERR_NOT_CONVERGED (39)
-    assert oracle.cg(csr, b, maxits=3)["status"] == ref.cg(n, r, c, v, b, maxits=3)["status"] == 0
-    assert oracle.cg(csr, b, maxits=3, rtol=1e-14)["status"] == ref.cg(n, r, c, v, b, maxits=3, rtol=1e-14)["status"] == 39
+    assert oracle.cg(csr, b, maxits=3)["status"] == pin["status__maxits"] == 0
+    assert oracle.cg(csr, b, maxits=3, rtol=1e-14)["status"] == pin["status__not_converged"] == 39
     # b = 0: r0 = 0, the scaled tolerance is 0, p.Ap = 0 -> indefinite (40)
     z = np.zeros(n)
-    assert oracle.cg(csr, z, maxits=3, rtol=1e-9)["status"] == ref.cg(n, r, c, v, z, maxits=3, rtol=1e-9)["status"] == 40
+    assert oracle.cg(csr, z, maxits=3, rtol=1e-9)["status"] == pin["status__indefinite"] == 40
     # already converged initial guess
     xs = np.random.default_rng(4).standard_normal(n)
     bb = oracle.dsymv(csr, 1.0, xs, 0.0, z)
     o = oracle.cg(csr, bb, x0=xs, maxits=10, atol=1e-6)
-    f = ref.cg(n, r, c, v, bb, x0=xs, maxits=10, atol=1e-6)
-    assert o["niterations"] == f["niterations"] == 0 and o["status"] == f["status"] == 0
+    assert o["niterations"] == pin["status__converged_x0_niterations"] == 0
+    assert o["status"] == pin["status__converged_x0"] == 0

@@ -108,43 +108,26 @@ def test_driver_solves_on_several_gpus(solver, method, oracle):
     assert int(lines[0].split()[0]) == N and np.abs(x - want["x"]).max() <= 1e-9 * np.abs(want["x"]).max()
 
 
-REFGPU = os.path.join(ROOT, "oracle", "_ref", "driver_ref", "acg-cuda-ref")
+STOCK = os.path.join(ROOT, "tests", "golden", "reference", "stock_gpu_27pt20.npz")
 
 
-@pytest.mark.gpu
 @pytest.mark.parametrize("solver,method", [("acg", "cg"), ("acg-pipelined", "cg_pipelined")])
 def test_stock_reference_gpu_solver_pins_the_oracle(solver, method, oracle):
     """The reference's OWN GPU solver (acg/cgcuda.c with cuSPARSE/cuBLAS, built unmodified
-    for sm_100a by tools/build_driver.sh) on the same file: the oracle restatement -- in
-    particular of pipelined CG, which the reference has no CPU version of -- must give the
-    same residual norms and solution after a fixed number of iterations.  Nothing of
-    libacgb200 is involved; a binary that cannot run on this box skips."""
-    if not os.path.exists(REFGPU):
-        pytest.skip("stock reference GPU binary not built (needs the reference tree at build time)")
+    for sm_100a by tools/build_driver.sh) on the same matrix, as stored from a run on a B200
+    (tools/make_reference_golden.py --stock-gpu): the oracle restatement -- in particular of
+    pipelined CG, which the reference has no CPU version of -- must give the same residual
+    norms and solution after a fixed number of iterations.  Nothing of libacgb200 is involved."""
+    g = np.load(STOCK)
     n, r, c, v = mg.stencil3d_27pt(20)
     csr = oracle.full_csr(n, r, c, v)
     its = 30
-    with tempfile.TemporaryDirectory() as d:
-        path = os.path.join(d, "A.mtx")
-        mtxio.write_symmetric(path, n, r, c, v, binary=True)
-        try:
-            p = subprocess.run([REFGPU, path, "--binary", "--solver", solver, "--max-iterations", str(its),
-                                "--residual-rtol", "0", "--warmup", "1", "--numfmt", "%.17g"],
-                               capture_output=True, text=True, timeout=300)
-        except subprocess.TimeoutExpired:
-            pytest.skip("stock reference GPU binary timed out on this box")
-    if p.returncode != 0:
-        pytest.skip("stock reference GPU binary does not run here: " + p.stderr[-300:])
-    rep = p.stderr
-    got_its = int(re.search(r"^\s*iterations: ([\d,]+)", rep, re.M).group(1).replace(",", ""))
-    rnrm2 = float(re.search(r"^\s*residual 2-norm: (\S+)", rep, re.M).group(1))
-    r0 = float(re.search(r"^\s*initial residual 2-norm: (\S+)", rep, re.M).group(1))
+    got_its, rnrm2, r0 = int(g[solver + "__niterations"]), float(g[solver + "__rnrm2"]), float(g[solver + "__r0nrm2"])
+    x = g[solver + "__x"]
     want = getattr(oracle, method)(csr, np.ones(n), maxits=its, rtol=0.0)
     assert got_its == want["niterations"] == its
     assert r0 == pytest.approx(want["r0nrm2"], rel=1e-13)
     assert rnrm2 / r0 == pytest.approx(want["rnrm2"] / want["r0nrm2"], rel=1e-8)
-    lines = [l for l in p.stdout.splitlines() if l and not l.startswith("%")]
-    x = np.array([float(t) for t in lines[1:]])
     assert len(x) == n
     assert np.abs(x - want["x"]).max() <= 1e-9 * np.abs(want["x"]).max()
 
